@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MNIST training images/s of the fused LeNet step on N B200s (BASELINE.json metric, config[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one pass of the hot path (forward + backward + packed-gradient reduction [+ all-reduce] + SGD update,
@@ -98,26 +98,25 @@ def measured_traffic(kernel, batch, steps):
         return None
 
 
+def dump_outputs(directory, eng):
+    """What the timed steps leave for a caller of Engine.train_steps, read back after the last one: the packed parameters
+    they updated, the packed gradient of the last step and the running sum of per-sample error norms.  The inputs depend
+    only on the arguments, so two builds of the project can be compared file for file."""
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "params.npy"), eng.get_params())
+    np.save(os.path.join(directory, "grads.npy"), eng.get_grads())
+    np.save(os.path.join(directory, "err_sum.npy"), np.array([eng.err_sum()], np.float64))
+
+
 def synthetic(n, seed):
     rng = np.random.default_rng(seed)
     return rng.integers(0, 256, (n, 784), dtype=np.uint8), rng.integers(0, 10, n, dtype=np.uint8)
 
 
-MNIST_DIR = os.path.join(ROOT, "oracle", "_ref", "data")
-
-
-def load_training_set(copies=5):
-    """The real MNIST training split (the four IDX files staged by oracle/Makefile next to the compiled reference) through
-    the engine's own loader, concatenated `copies` times so that the device-resident set (235 MB) is larger than the
-    126 MB L2 -- every step then reads its batch from HBM.  Falls back to synthetic MNIST-shaped bytes when the files
-    are absent.  Returns (images u8 [n,784], labels u8 [n], description)."""
-    img, lab = os.path.join(MNIST_DIR, "train-images.idx3-ubyte"), os.path.join(MNIST_DIR, "train-labels.idx1-ubyte")
-    if os.path.exists(img) and os.path.exists(lab):
-        import pcnn_loader
-        rc, images, labels = pcnn_loader.load().mnist_load_u8(img, lab)
-        if rc == 0:
-            return (np.ascontiguousarray(np.tile(images, (copies, 1))), np.ascontiguousarray(np.tile(labels, copies)),
-                    f"mnist (train split, 60000 images x {copies} concatenated copies = {copies * 47.04:.0f} MB)")
+def load_training_set():
+    """Seeded synthetic MNIST-shaped bytes, the same on every run whatever else lies in the tree, so that runs of two builds
+    see identical inputs; the device-resident set (205 MB) is larger than the 126 MB L2, so every step reads its batch
+    from HBM.  Returns (images u8 [n,784], labels u8 [n], description)."""
     imgs, labs = synthetic(DATASET_IMAGES, 7)
     return imgs, labs, "synthetic"
 
@@ -155,7 +154,7 @@ def _ref_worker(args):
             pass
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import oracle_lib as O
-    imgs, labs, _ = load_training_set(copies=1)
+    imgs, labs, _ = load_training_set()
     lo = (wid * n) % max(1, imgs.shape[0] - n)
     imgs, labs = np.ascontiguousarray(imgs[lo:lo + n]), np.ascontiguousarray(labs[lo:lo + n])
     ref = O.reference(native=native)
@@ -189,7 +188,7 @@ def run_reference_arm(a):
     import oracle_lib as O
     kind = "reference" if O.reference() is not None else "port"
     cores, aff, why = host_cores()
-    _, _, data = load_training_set(copies=1)
+    _, _, data = load_training_set()
     # bounded sample: ~60 s of CPU work in total at ~4.4 k img/s/core (BASELINE.md section 2)
     n_per_step = int(max(8, min(4096, 60.0 * 4400 / max(1, a.steps + a.warmup))))
     value, secs = cpu_reference_throughput(cores, aff, n_per_step, a.steps, a.warmup)
@@ -295,8 +294,7 @@ def run_ours(a):
     eng = pkg.Engine(local, stream.cuda_stream)
     B, K, W = a.batch, a.steps, max(a.warmup, 3)
 
-    # the training set (real MNIST x5 when staged, else synthetic bytes), identical on every rank: ranks read disjoint
-    # windows of every global batch
+    # the training set, identical on every rank: ranks read disjoint windows of every global batch
     imgs, labs, data_desc = load_training_set()
     n_data = imgs.shape[0]
     eng.dataset_upload(pkg.TRAIN_SET, imgs, labs)
@@ -427,6 +425,8 @@ def run_ours(a):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = K * B * world / (ms * 1e-3)
+    if a.dump_outputs and rank == 0:         # replicas are identical after every step
+        dump_outputs(a.dump_outputs, eng)
 
     # ---- e2e: pinned host buffers through the public host API (single-GPU entry point; per-rank shard when N > 1)
     K2 = min(K, 8192)                        # bounds the pinned host buffer (8192 steps x 256 x 784 B = 1.6 GB)
@@ -593,7 +593,11 @@ def main():
     ap.add_argument("--mode", default="auto", choices=["auto", "graph", "persistent"],
                     help="auto/persistent: one cooperative kernel runs all K steps (N > 1: in-kernel NVLink exchange); "
                          "graph: per-step kernels replayed from CUDA graphs (N > 1: ncclAllReduce per step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what they computed as DIR/params.npy, grads.npy, err_sum.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if a.impl == "reference":
         run_reference_arm(a)
     else:

@@ -9,10 +9,18 @@ output of the reference's own code on real MNIST bytes:
   reference_vectors.npz  seed-1 parameters, per-sample activations / backward buffers, parameter states after
                          1, 1000 and 60000 steps, per-step error norms, classifications
   reference_scalars.json the SURVEY.md Appendix B numbers re-measured here (err, error rate, sums, FNV hashes)
+  reference_ops.json     SHA-256 of every operator output of the reference on seeded random inputs, and of its
+                         parameters after the seed-1 redraw
+  reference_fixture_epoch.npz  the reference's own driver and learn loop on the stored samples shaped as a full epoch
+                         (oracle_lib.fixture_splits): printed lines, mean error, test mismatches, final parameters
+The last two let the tests compare with the reference where it cannot be built; `--selfcontained` writes only them.
 """
 import json
 import os
+import re
+import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -108,5 +116,47 @@ def main():
     print(json.dumps(sc, indent=1, sort_keys=True))
 
 
+OPS_TRIALS, OPS_SEED = 5, 1234
+
+
+def selfcontained():
+    """Must run on a freshly loaded reference: its first record is the static constructors' parameter state."""
+    ref = O.reference()
+    if ref is None:
+        raise SystemExit("oracle/_ref/libref_seq.so missing: run `make -C oracle` where the reference sources exist")
+    p = np.empty(O.NPARAM, np.float32)
+    ref.ref_get_params(O.fp(p))
+    static = O.digest(p)
+    rng = np.random.default_rng(OPS_SEED)
+    trials = [{name: O.digest(a) for name, a in O.op_chain(ref, "ref_", rng, t)} for t in range(OPS_TRIALS)]
+    ref.ref_reset_params()
+    ref.ref_get_params(O.fp(p))
+    ops = {"seed": OPS_SEED, "trials": trials, "params_static_constructors": static, "params_after_reset": O.digest(p),
+           "sizeof_mnist_data": int(ref.ref_sizeof_mnist_data())}
+    with open(O.REF_OPS, "w") as f:
+        json.dump(ops, f, indent=1)
+
+    subset = np.load(os.path.join(O.GOLDEN, "mnist_subset.npz"))
+    tr, trl, te, tel = O.fixture_splits(subset)
+    ref.ref_reset_params()
+    secs = np.zeros(1, np.float64)
+    err = ref.ref_learn_loop_u8(O.u8p(tr.reshape(-1)), O.u8p(trl), len(trl), O.dp(secs))
+    ref.ref_get_params(O.fp(p))
+    wrong = int(ref.ref_test_u8(O.u8p(te.reshape(-1)), O.u8p(tel), len(tel)))
+    # the reference's own driver (Sequential/Main.cpp, unmodified) on the same four files prints the same two results
+    with tempfile.TemporaryDirectory() as tmp:
+        O.write_fixture_data(os.path.join(tmp, "data"), subset)
+        out = subprocess.run([os.path.join(O.ROOT, "oracle", "_ref", "seq_main")], cwd=tmp, capture_output=True, text=True,
+                             check=True).stdout
+    err_printed = re.search(r"error: (\S+), time_on_cpu", out).group(1)
+    rate_printed = re.search(r"Error Rate: (\S+)%", out).group(1)
+    assert err_printed == "%e" % err and rate_printed == "%.2f" % (wrong / len(tel) * 100.0), (out, err, wrong)
+    np.savez_compressed(O.REF_EPOCH, epoch_err=np.float32(err), test_wrong=np.int64(wrong), test_count=np.int64(len(tel)),
+                        err_printed=np.array(err_printed), rate_printed=np.array(rate_printed), params_after_epoch=p)
+    print(json.dumps({"epoch_err": float(err), "err_printed": err_printed, "test_wrong": wrong, "rate_printed": rate_printed}))
+
+
 if __name__ == "__main__":
-    main()
+    selfcontained()
+    if "--selfcontained" not in sys.argv[1:]:
+        main()

@@ -5,6 +5,7 @@
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs import this module.
 """
 import ctypes as C
+import hashlib
 import os
 import numpy as np
 
@@ -244,3 +245,95 @@ def full_mnist():
     if not all(os.path.exists(x) for x in f):
         return None
     return read_idx_images(f[0]), read_idx_labels(f[1]), read_idx_images(f[2]), read_idx_labels(f[3])
+
+
+# ---------------------------------------------------------------- stand-ins for the reference's runs on the full dataset
+EPOCH_STEPS = 60000     # one epoch of Main.cpp's learn() at batch 1 on the MNIST training split
+
+
+def fixture_splits(subset):
+    """The stored MNIST samples (tests/golden/mnist_subset.npz) shaped like the reference's run: a 60,000-sample training
+    split made of the 1,024 stored training samples repeated in order, and the 256 stored test samples as the test split."""
+    tr = np.resize(subset["train_u8"], (EPOCH_STEPS, 784))
+    trl = np.resize(subset["train_labels"], EPOCH_STEPS)
+    return tr, trl, np.ascontiguousarray(subset["test_u8"]), np.ascontiguousarray(subset["test_labels"])
+
+
+def write_idx(directory, images, labels, stem):
+    """`stem`-images.idx3-ubyte and `stem`-labels.idx1-ubyte in the MNIST IDX format mnist.h reads."""
+    os.makedirs(directory, exist_ok=True)
+    with open(os.path.join(directory, f"{stem}-images.idx3-ubyte"), "wb") as f:
+        f.write(np.array([2051, len(images), 28, 28], ">u4").tobytes())
+        f.write(np.ascontiguousarray(images, np.uint8).tobytes())
+    with open(os.path.join(directory, f"{stem}-labels.idx1-ubyte"), "wb") as f:
+        f.write(np.array([2049, len(labels)], ">u4").tobytes())
+        f.write(np.ascontiguousarray(labels, np.uint8).tobytes())
+
+
+def write_fixture_data(directory, subset):
+    """The four IDX files Main.cpp's loaddata() opens, holding fixture_splits(subset)."""
+    tr, trl, te, tel = fixture_splits(subset)
+    write_idx(directory, tr, trl, "train")
+    write_idx(directory, te, tel, "t10k")
+    return directory
+
+
+REF_EPOCH = os.path.join(GOLDEN, "reference_fixture_epoch.npz")
+REF_OPS = os.path.join(GOLDEN, "reference_ops.json")
+
+
+def reference_fixture_epoch():
+    """What the reference computed on fixture_splits() (oracle/gen_golden.py): its driver's printed lines, the mean error of
+    the epoch, the mismatches of its test() and its parameters after the epoch."""
+    return dict(np.load(REF_EPOCH))
+
+
+def digest(a):
+    return hashlib.sha256(np.ascontiguousarray(a, np.float32).tobytes()).hexdigest()
+
+
+# the reference's spelling where the oracle's entry point is named differently
+_REF_OP_NAMES = {"make_error": "makeError", "vector_norm": "vectorNorm"}
+
+
+def op_chain(L, prefix, rng, label):
+    """Every layer.h operator once, on inputs drawn from `rng`, each fed with the outputs of the ones before it as Main.cpp's
+    forward and backward passes feed them.  L is the oracle (prefix "orc_") or the compiled reference ("ref_").  Returns
+    [(name, float32 array)] in call order, the drawn inputs first."""
+    def op(name, *args):
+        return getattr(L, prefix + (_REF_OP_NAMES.get(name, name) if prefix == "ref_" else name))(*args)
+
+    def r(*shape, lo=-1.0, hi=1.0):
+        return np.ascontiguousarray(rng.uniform(lo, hi, shape).astype(np.float32))
+
+    inp, w1, b1 = r(784, lo=0, hi=1), r(150, lo=-.5, hi=.5), r(6, lo=-.5, hi=.5)
+    w2, b2 = r(16), r(1)
+    x216, wf, bf = r(216, lo=0, hi=1), r(2160), r(10)
+    out10 = r(10, lo=0, hi=1)
+    z = lambda n: np.zeros(n, np.float32)  # noqa: E731
+    o1, s1, p1, f1, e1 = z(3456), z(3456), z(216), z(10), z(10)
+    op("fp_c1", fp(inp), fp(o1), fp(w1), fp(b1))
+    op("apply_step_function", fp(o1), fp(s1), 3456)
+    op("fp_s1", fp(s1), fp(p1), fp(w2), fp(b2))
+    op("fp_preact_f", fp(x216), fp(f1), fp(wf))
+    op("fp_bias_f", fp(f1), fp(bf))
+    op("make_error", fp(e1), fp(out10), label, 10)
+    norm = np.array([op("vector_norm", fp(e1), 10)], np.float32)
+    d1, q1, t1, g1, u1, v1, h1 = z(2160), z(216), z(216), z(16), z(3456), z(3456), z(150)
+    bfa, b2a, b1a, wfa = bf.copy(), b2.copy(), b1.copy(), wf.copy()
+    op("bp_weight_f", fp(d1), fp(e1), fp(x216))
+    op("bp_bias_f", fp(bfa), fp(e1))
+    op("bp_output_s1", fp(q1), fp(wf), fp(e1))
+    op("bp_preact_s1", fp(t1), fp(q1), fp(p1))
+    op("bp_weight_s1", fp(g1), fp(t1), fp(s1))
+    op("bp_bias_s1", fp(b2a), fp(t1))
+    op("bp_output_c1", fp(u1), fp(w2), fp(t1))
+    op("bp_preact_c1", fp(v1), fp(u1), fp(o1))
+    op("bp_weight_c1", fp(h1), fp(v1), fp(inp))
+    op("bp_bias_c1", fp(b1a), fp(v1))
+    op("apply_grad", fp(wfa), fp(d1), 2160)
+    inputs = np.concatenate([inp, w1, b1, w2, b2, x216, wf, bf, out10])
+    return [("inputs", inputs), ("fp_c1", o1), ("apply_step_function", s1), ("fp_s1", p1), ("fp_preact_f + fp_bias_f", f1),
+            ("makeError", e1), ("vectorNorm", norm), ("bp_weight_f", d1), ("bp_bias_f", bfa), ("bp_output_s1", q1),
+            ("bp_preact_s1", t1), ("bp_weight_s1", g1), ("bp_bias_s1", b2a), ("bp_output_c1", u1), ("bp_preact_c1", v1),
+            ("bp_weight_c1", h1), ("bp_bias_c1", b1a), ("apply_grad", wfa)]

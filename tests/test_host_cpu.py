@@ -79,13 +79,14 @@ def test_mnist_loader_return_codes_follow_mnist_h(pkg, golden, tmp_path):
     assert pkg.mnist_load_u8(*_write_idx(tmp, imgs, labs, dims=(28, 27)))[0] == -2    # mnist.h:128-131
 
 
-def test_mnist_loader_reads_the_real_idx_files(pkg, golden):
-    d = O.REF_DATA
-    if not os.path.exists(os.path.join(d, "t10k-images.idx3-ubyte")):
-        pytest.skip("full MNIST not staged under oracle/_ref/data")
-    rc, a, b = pkg.mnist_load_u8(os.path.join(d, "t10k-images.idx3-ubyte"), os.path.join(d, "t10k-labels.idx1-ubyte"))
+def test_mnist_loader_reads_the_real_idx_files(pkg, golden, tmp_path):
+    """IDX files of the MNIST test split's size and header (10,000 images of 28 x 28), filled with the 256 stored real test
+    samples repeated in order."""
+    te, tel = np.resize(golden["test_u8"], (10000, 784)), np.resize(golden["test_labels"], 10000)
+    O.write_idx(str(tmp_path), te, tel, "t10k")
+    rc, a, b = pkg.mnist_load_u8(str(tmp_path / "t10k-images.idx3-ubyte"), str(tmp_path / "t10k-labels.idx1-ubyte"))
     assert rc == 0 and a.shape == (10000, 784)
-    assert np.array_equal(a[:256], golden["test_u8"]) and np.array_equal(b[:256], golden["test_labels"])
+    assert np.array_equal(a, te) and np.array_equal(b, tel)
 
 
 def test_sharding_covers_the_global_batch_exactly(pkg):
