@@ -275,7 +275,7 @@ int pcnn_conv_tc_plan_create(pcnn_ctx *ctx, int N, int H, int W, int C, int K, i
                              int act, const float *filt_host, const float *bias_host, pcnn_conv_plan **plan_out);
 /* the same with a window step of `stride` (1..4) in both directions (SURVEY.md 8f row 4): y [N][(H-R)/stride+1][(W-S)/stride+1][K];
  * rows per image (image_rows, or H) must be a multiple of the stride; the pixel block then needs ((Qt-1)*stride+S)*C <= 32.
- * Backward passes of strided convolutions are not built. */
+ * Its backward passes are pcnn_conv_wgrad_strided / pcnn_conv_dgrad_strided below. */
 int pcnn_conv_tc_plan_create_strided(pcnn_ctx *ctx, int N, int H, int W, int C, int K, int R, int S, int stride, int row_pitch,
                                      int image_rows, int act, const float *filt_host, const float *bias_host,
                                      pcnn_conv_plan **plan_out);
@@ -288,6 +288,18 @@ int pcnn_conv_wgrad(pcnn_ctx *ctx, const void *x_bf16_dev, const void *dy_bf16_d
                     int K, int R, int S, int row_pitch, int image_rows);
 int pcnn_conv_dgrad(pcnn_ctx *ctx, const void *dy_bf16_dev, const float *filt_f32_dev, void *dx_bf16_dev, int N, int H, int W,
                     int C, int K, int R, int S, int row_pitch, int image_rows);
+/* The same with a window step of `stride` (1..4, else PCNN_ERR_ARG) in both directions: dy [N][(H-R)/stride+1][(W-S)/stride+1][K],
+ *     dw[k][r][s][c] = sum dy[n][p][q][k] * x[n][p*stride+r][q*stride+s][c]
+ *     dx[n][h][w][c] = sum over (h-r) % stride == 0, (w-s) % stride == 0 of dy[n][(h-r)/stride][(w-s)/stride][k] * f[k][r][s][c].
+ * Rows per image need not be a multiple of the stride.  Every dx element is written, rows and columns no tap reaches as 0.
+ * stride = 1 is pcnn_conv_wgrad / pcnn_conv_dgrad.  The tensor-core weight gradient needs ((RB-1)*stride + R)*S*C <= 64 for some
+ * RB >= 1 and a row pitch that is a multiple of 8 elements; the tensor-core input gradient is built for 3x3 taps with C in
+ * {1,2,3,4,8}, 5x5 with C in {1,3} and 7x7 with C = 1 at strides 1 and 2, 3x3 with C in {1,2,3} at stride 3, 3x3x3 and 5x5x1 at
+ * stride 4.  Other shapes are refused as for stride 1 (see pcnn_conv_bwd_select). */
+int pcnn_conv_wgrad_strided(pcnn_ctx *ctx, const void *x_bf16_dev, const void *dy_bf16_dev, float *dw_f32_dev, int N, int H, int W,
+                            int C, int K, int R, int S, int stride, int row_pitch, int image_rows);
+int pcnn_conv_dgrad_strided(pcnn_ctx *ctx, const void *dy_bf16_dev, const float *filt_f32_dev, void *dx_bf16_dev, int N, int H, int W,
+                            int C, int K, int R, int S, int stride, int row_pitch, int image_rows);
 /* Which kernels pcnn_conv_wgrad / pcnn_conv_dgrad may use.  PCNN_CONV_BWD_TENSOR (default): the tcgen05 kernels only (any filter
  * count up to 256: counts that are not a multiple of 64 are zero-padded to one in an extra pass over dy) -- a shape they
  * cannot take is an ERROR (PCNN_ERR_ARG naming the restriction), never a silent detour.  PCNN_CONV_BWD_REFERENCE: the
@@ -299,6 +311,8 @@ int pcnn_conv_bwd_select(pcnn_ctx *ctx, int path);
  * out9 = { wgrad on tensor cores, dy rows per tile, pixels per tile, stages,
  *          dgrad on tensor cores, column strips, output pixels per lane quarter, TMEM slot groups in flight, stages } */
 int pcnn_conv_bwd_plan_info(int N, int H, int W, int C, int K, int R, int S, int *out9);
+/* the same for a window step of `stride` (1..4, else PCNN_ERR_ARG); out9[6] counts dx columns per lane quarter */
+int pcnn_conv_bwd_plan_info_strided(int N, int H, int W, int C, int K, int R, int S, int stride, int *out9);
 /* Zero padding for the valid-padding kernels above (SURVEY.md 8f row 4): pcnn_pad_nhwc_bf16 embeds dense [N][H][W][C] images into
  * a zeroed canvas [N][dst_image_rows][dst_row_pitch] at row offset pad_h, pixel offset pad_w (0 = the tight canvas
  * [H + 2 pad_h][(W + 2 pad_w) * C]); a "same" convolution is pad -> pcnn_conv_tc_fwd, its input gradient is

@@ -117,10 +117,13 @@ _SIG = {
     "pcnn_conv_tc_fwd": [_vp, _vp, _vp, _vp],
     "pcnn_f32_to_bf16_rows": [_vp, _vp, _vp, _l, _i, _i],
     "pcnn_conv_bwd_plan_info": [_i, _i, _i, _i, _i, _i, _i, _vp],
+    "pcnn_conv_bwd_plan_info_strided": [_i, _i, _i, _i, _i, _i, _i, _i, _vp],
     "pcnn_pad_nhwc_bf16": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i],
     "pcnn_crop_nhwc_bf16": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i],
     "pcnn_conv_wgrad": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i],
     "pcnn_conv_dgrad": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i],
+    "pcnn_conv_wgrad_strided": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i],
+    "pcnn_conv_dgrad_strided": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i],
 }
 _RESTYPE = {"pcnn_last_error_string": C.c_char_p, "pcnn_mnist_free": None}
 

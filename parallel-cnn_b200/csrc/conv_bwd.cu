@@ -7,21 +7,24 @@
 // FMA-pipe kernels (used by the tests to check both paths against the oracle).
 //   wgrad  dw[k][r][s][c] = sum_{n,p,q} dy[n][p][q][k] * x[n][p+r][q+s][c]          [ref: layer.h:371-395 without the /576]
 //   dgrad  dx[n][h][w][c] = sum_{k,r,s} dy[n][h-r][w-s][k] * f[k][r][s][c]          (the reference never needs it: c1 is the first layer)
+// The _strided entry points take a window step st in 1..4 (the forward plan's pcnn_conv_tc_plan_create_strided): x[n][p*st+r][q*st+s][c]
+// in the weight gradient, dy[n][(h-r)/st][(w-s)/st][k] over (h-r) % st == 0, (w-s) % st == 0 in the input gradient; the
+// stride-1 entry points are that case.
 #include "pcnn_internal.h"
 
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
 // conv_dgrad_tc.cu
-bool pcnn_conv_dgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, const void *dy);
+bool pcnn_conv_dgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, int stride, const void *dy);
 int pcnn_conv_dgrad_rows(pcnn_ctx *ctx, const void *dy_bf16, const float *filt_f32_dev, void *dx_bf16, int N, int H, int W, int C, int K,
-                         int R, int S, int row_pitch, int image_rows, int dy_channels = 0);
+                         int R, int S, int stride, int row_pitch, int image_rows, int dy_channels = 0);
 // conv_wgrad_tc.cu
-bool pcnn_conv_wgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, int row_pitch, const void *x, const void *dy);
+bool pcnn_conv_wgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, int stride, int row_pitch, const void *x, const void *dy);
 int pcnn_conv_wgrad_rows(pcnn_ctx *ctx, const void *x_bf16, const void *dy_bf16, float *dw_f32, int N, int H, int W, int C, int K,
-                         int R, int S, int row_pitch, int image_rows, int dy_channels = 0);
-void pcnn_conv_dgrad_rows_info(int H, int W, int C, int K, int R, int S, int *out4);
-void pcnn_conv_wgrad_rows_info(int H, int W, int C, int K, int R, int S, int *out4);
+                         int R, int S, int stride, int row_pitch, int image_rows, int dy_channels = 0);
+void pcnn_conv_dgrad_rows_info(int H, int W, int C, int K, int R, int S, int stride, int *out4);
+void pcnn_conv_wgrad_rows_info(int H, int W, int C, int K, int R, int S, int stride, int *out4);
 
 namespace {
 
@@ -32,6 +35,7 @@ struct ConvShape {
     int N, H, W, C, K, R, S, P, Q;
     int row_pitch;                    // elements between rows of x
     int image_rows;                   // rows between images of x
+    int stride;                       // window step in both directions
 };
 
 __device__ __forceinline__ float bf(const __nv_bfloat16 *p) { return __bfloat162float(*p); }
@@ -58,12 +62,13 @@ __global__ void __launch_bounds__(WG_THREADS) k_conv_wgrad_partial(const __nv_bf
     const long rows = (long)s.N * s.P;
     for (long row = blockIdx.x; row < rows; row += gridDim.x) {
         const int n = (int)(row / s.P), p = (int)(row % s.P);
-        const __nv_bfloat16 *xr = x + ((long)n * s.image_rows + p) * s.row_pitch;
+        const __nv_bfloat16 *xr = x + ((long)n * s.image_rows + p * s.stride) * s.row_pitch;
         const __nv_bfloat16 *dr = dy + row * s.Q * s.K;
+        const int xstep = s.stride * s.C;
         for (int q = 0; q < s.Q; ++q) {
 #pragma unroll
             for (int i = 0; i < WG_MAXO; ++i)
-                if (xoff[i] >= 0) acc[i] = fmaf(bf(dr + q * s.K + k[i]), bf(xr + q * s.C + xoff[i]), acc[i]);
+                if (xoff[i] >= 0) acc[i] = fmaf(bf(dr + q * s.K + k[i]), bf(xr + q * xstep + xoff[i]), acc[i]);
         }
     }
 #pragma unroll
@@ -99,11 +104,13 @@ __global__ void __launch_bounds__(256) k_conv_dgrad(const __nv_bfloat16 *__restr
         const int n = (int)(idx / ((long)s.C * s.W * s.H));
         float acc = 0.0f;
         for (int r = 0; r < s.R; ++r) {
-            const int p = h - r;
-            if (p < 0 || p >= s.P) continue;
+            if (h - r < 0 || (h - r) % s.stride) continue;
+            const int p = (h - r) / s.stride;
+            if (p >= s.P) continue;
             for (int ss = 0; ss < s.S; ++ss) {
-                const int q = w - ss;
-                if (q < 0 || q >= s.Q) continue;
+                if (w - ss < 0 || (w - ss) % s.stride) continue;
+                const int q = (w - ss) / s.stride;
+                if (q >= s.Q) continue;
                 const __nv_bfloat16 *d = dy + (((long)n * s.P + p) * s.Q + q) * s.K;
                 const float *fp = f + ((long)r * s.S + ss) * s.C + c;
                 for (int k = 0; k < s.K; ++k) acc = fmaf(bf(d + k), fp[(long)k * s.R * s.S * s.C], acc);
@@ -166,27 +173,27 @@ int pad_dy(pcnn_ctx *ctx, const void *dy_bf16, long rows, int K, int Kp, size_t 
     return PCNN_OK;
 }
 
-int check_shape(const char *fn, int N, int H, int W, int C, int K, int R, int S, int row_pitch, int image_rows, ConvShape *out) {
+int check_shape(const char *fn, int N, int H, int W, int C, int K, int R, int S, int stride, int row_pitch, int image_rows, ConvShape *out) {
     PCNN_REQUIRE(N > 0 && C > 0 && K > 0 && R > 0 && S > 0 && H >= R && W >= S, PCNN_ERR_ARG, "%s: bad shape", fn);
+    PCNN_REQUIRE(stride >= 1 && stride <= 4, PCNN_ERR_ARG, "%s: stride %d outside 1..4", fn, stride);
     if (row_pitch <= 0) row_pitch = W * C;
     if (image_rows <= 0) image_rows = H;
     PCNN_REQUIRE(row_pitch >= W * C && image_rows >= H, PCNN_ERR_ARG, "%s: pitches smaller than the image", fn);
     out->N = N; out->H = H; out->W = W; out->C = C; out->K = K; out->R = R; out->S = S;
-    out->P = H - R + 1; out->Q = W - S + 1; out->row_pitch = row_pitch; out->image_rows = image_rows;
+    out->P = (H - R) / stride + 1; out->Q = (W - S) / stride + 1; out->row_pitch = row_pitch; out->image_rows = image_rows;
+    out->stride = stride;
     return PCNN_OK;
 }
 
-}  // namespace
-
-extern "C" int pcnn_conv_wgrad(pcnn_ctx *ctx, const void *x_bf16, const void *dy_bf16, float *dw_f32, int N, int H, int W, int C,
-                               int K, int R, int S, int row_pitch, int image_rows) {
-    PCNN_REQUIRE(ctx && x_bf16 && dy_bf16 && dw_f32, PCNN_ERR_ARG, "pcnn_conv_wgrad: NULL argument");
+int conv_wgrad(const char *fn, pcnn_ctx *ctx, const void *x_bf16, const void *dy_bf16, float *dw_f32, int N, int H, int W, int C, int K, int R,
+               int S, int stride, int row_pitch, int image_rows) {
+    PCNN_REQUIRE(ctx && x_bf16 && dy_bf16 && dw_f32, PCNN_ERR_ARG, "%s: NULL argument", fn);
     ConvShape s;
-    int rc = check_shape("pcnn_conv_wgrad", N, H, W, C, K, R, S, row_pitch, image_rows, &s);
+    int rc = check_shape(fn, N, H, W, C, K, R, S, stride, row_pitch, image_rows, &s);
     if (rc) return rc;
     if (ctx->conv_bwd_path == PCNN_CONV_BWD_TENSOR) {
         const int Kp = (K + 63) / 64 * 64;
-        if (K % 64 && Kp <= 256 && pcnn_conv_wgrad_rows_ok(N, H, W, C, Kp, R, S, s.row_pitch, x_bf16, nullptr)) {
+        if (K % 64 && Kp <= 256 && pcnn_conv_wgrad_rows_ok(N, H, W, C, Kp, R, S, stride, s.row_pitch, x_bf16, nullptr)) {
             pcnn_device_guard g(ctx->device);
             __nv_bfloat16 *dyp = nullptr;
             void *dwp = nullptr;
@@ -202,19 +209,20 @@ extern "C" int pcnn_conv_wgrad(pcnn_ctx *ctx, const void *x_bf16, const void *dy
                 return rc;
             }
             if ((rc = pcnn_conv_wgrad_rows(ctx, x_bf16, in_place ? dy_bf16 : dyp, reinterpret_cast<float *>(dwp), N, H, W, C, Kp, R, S,
-                                           s.row_pitch, s.image_rows, in_place ? K : 0)))
+                                           stride, s.row_pitch, s.image_rows, in_place ? K : 0)))
                 return rc;
             PCNN_CUDA(cudaMemcpyAsync(dw_f32, dwp, (size_t)K * rsc * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));   // filters 0..K-1
             return PCNN_OK;
         }
-        PCNN_REQUIRE(pcnn_conv_wgrad_rows_ok(N, H, W, C, K, R, S, s.row_pitch, x_bf16, dy_bf16), PCNN_ERR_ARG,
-                     "pcnn_conv_wgrad: no tensor-core kernel for C = %d, K = %d, %dx%d taps (needs K <= 256 -- padded to a multiple of 64 --, (RB + R - 1) * S * C <= 64, "
-                     "16-byte aligned operands); the FMA-pipe reference kernels (~1 %% of the HBM roofline) must be selected explicitly with "
-                     "pcnn_conv_bwd_select(ctx, PCNN_CONV_BWD_REFERENCE)", C, K, R, S);
-        return pcnn_conv_wgrad_rows(ctx, x_bf16, dy_bf16, dw_f32, N, H, W, C, K, R, S, s.row_pitch, s.image_rows);
+        PCNN_REQUIRE(pcnn_conv_wgrad_rows_ok(N, H, W, C, K, R, S, stride, s.row_pitch, x_bf16, dy_bf16), PCNN_ERR_ARG,
+                     "%s: no tensor-core kernel for C = %d, K = %d, %dx%d taps, stride %d (needs K <= 256 -- padded to a multiple of 64 --, "
+                     "((RB - 1) * stride + R) * S * C <= 64, a row pitch that is a multiple of 8 elements, 16-byte aligned operands); the FMA-pipe "
+                     "reference kernels (~1 %% of the HBM roofline) must be selected explicitly with pcnn_conv_bwd_select(ctx, PCNN_CONV_BWD_REFERENCE)",
+                     fn, C, K, R, S, stride);
+        return pcnn_conv_wgrad_rows(ctx, x_bf16, dy_bf16, dw_f32, N, H, W, C, K, R, S, stride, s.row_pitch, s.image_rows);
     }
     const int nout = K * R * S * C;
-    PCNN_REQUIRE(nout <= WG_THREADS * WG_MAXO, PCNN_ERR_ARG, "pcnn_conv_wgrad: K*R*S*C = %d exceeds %d", nout, WG_THREADS * WG_MAXO);
+    PCNN_REQUIRE(nout <= WG_THREADS * WG_MAXO, PCNN_ERR_ARG, "%s: K*R*S*C = %d exceeds %d", fn, nout, WG_THREADS * WG_MAXO);
     pcnn_device_guard g(ctx->device);
     const long rows = (long)N * s.P;
     int grid = (int)(rows < (long)ctx->sm_count * 8 ? rows : (long)ctx->sm_count * 8);
@@ -228,15 +236,15 @@ extern "C" int pcnn_conv_wgrad(pcnn_ctx *ctx, const void *x_bf16, const void *dy
     return PCNN_OK;
 }
 
-extern "C" int pcnn_conv_dgrad(pcnn_ctx *ctx, const void *dy_bf16, const float *filt_f32_dev, void *dx_bf16, int N, int H, int W,
-                               int C, int K, int R, int S, int row_pitch, int image_rows) {
-    PCNN_REQUIRE(ctx && dy_bf16 && filt_f32_dev && dx_bf16, PCNN_ERR_ARG, "pcnn_conv_dgrad: NULL argument");
+int conv_dgrad(const char *fn, pcnn_ctx *ctx, const void *dy_bf16, const float *filt_f32_dev, void *dx_bf16, int N, int H, int W, int C, int K,
+               int R, int S, int stride, int row_pitch, int image_rows) {
+    PCNN_REQUIRE(ctx && dy_bf16 && filt_f32_dev && dx_bf16, PCNN_ERR_ARG, "%s: NULL argument", fn);
     ConvShape s;
-    int rc = check_shape("pcnn_conv_dgrad", N, H, W, C, K, R, S, row_pitch, image_rows, &s);
+    int rc = check_shape(fn, N, H, W, C, K, R, S, stride, row_pitch, image_rows, &s);
     if (rc) return rc;
     if (ctx->conv_bwd_path == PCNN_CONV_BWD_TENSOR) {
         const int Kp = (K + 63) / 64 * 64;
-        if (K % 64 && Kp <= 256 && pcnn_conv_dgrad_rows_ok(N, H, W, C, Kp, R, S, nullptr)) {
+        if (K % 64 && Kp <= 256 && pcnn_conv_dgrad_rows_ok(N, H, W, C, Kp, R, S, stride, nullptr)) {
             pcnn_device_guard g(ctx->device);
             __nv_bfloat16 *dyp = nullptr;
             void *fp = nullptr;
@@ -252,13 +260,14 @@ extern "C" int pcnn_conv_dgrad(pcnn_ctx *ctx, const void *dy_bf16, const float *
             k_pad_filters_f32<<<(Kp * rsc + 255) / 256, 256, 0, ctx->stream>>>(filt_f32_dev, reinterpret_cast<float *>(fp), K, Kp, rsc);
             PCNN_CHECK_LAUNCH(ctx);
             return pcnn_conv_dgrad_rows(ctx, in_place ? dy_bf16 : dyp, reinterpret_cast<const float *>(fp), dx_bf16, N, H, W, C, Kp, R, S,
-                                        s.row_pitch, s.image_rows, in_place ? K : 0);
+                                        stride, s.row_pitch, s.image_rows, in_place ? K : 0);
         }
-        PCNN_REQUIRE(pcnn_conv_dgrad_rows_ok(N, H, W, C, K, R, S, dy_bf16), PCNN_ERR_ARG,
-                     "pcnn_conv_dgrad: no tensor-core kernel for C = %d, K = %d, %dx%d taps (needs K <= 256 -- padded to a multiple of 64 -- and 3x3 taps with C in "
-                     "{1,2,3,4,8}, 5x5 with C in {1,3} or 7x7 with C = 1); the FMA-pipe reference kernels (~1 %% of the HBM roofline) must be "
-                     "selected explicitly with pcnn_conv_bwd_select(ctx, PCNN_CONV_BWD_REFERENCE)", C, K, R, S);
-        return pcnn_conv_dgrad_rows(ctx, dy_bf16, filt_f32_dev, dx_bf16, N, H, W, C, K, R, S, s.row_pitch, s.image_rows);
+        PCNN_REQUIRE(pcnn_conv_dgrad_rows_ok(N, H, W, C, K, R, S, stride, dy_bf16), PCNN_ERR_ARG,
+                     "%s: no tensor-core kernel for C = %d, K = %d, %dx%d taps, stride %d (needs K <= 256 -- padded to a multiple of 64 -- and, "
+                     "at strides 1 and 2, 3x3 taps with C in {1,2,3,4,8}, 5x5 with C in {1,3} or 7x7 with C = 1; at stride 3, 3x3 with C in "
+                     "{1,2,3}; at stride 4, 3x3 with C = 3 or 5x5 with C = 1); the FMA-pipe reference kernels (~1 %% of the HBM roofline) must "
+                     "be selected explicitly with pcnn_conv_bwd_select(ctx, PCNN_CONV_BWD_REFERENCE)", fn, C, K, R, S, stride);
+        return pcnn_conv_dgrad_rows(ctx, dy_bf16, filt_f32_dev, dx_bf16, N, H, W, C, K, R, S, stride, s.row_pitch, s.image_rows);
     }
     pcnn_device_guard g(ctx->device);
     const long total = (long)N * H * W * C;
@@ -268,6 +277,28 @@ extern "C" int pcnn_conv_dgrad(pcnn_ctx *ctx, const void *dy_bf16, const float *
                                                       reinterpret_cast<__nv_bfloat16 *>(dx_bf16), s);
     PCNN_CHECK_LAUNCH(ctx);
     return PCNN_OK;
+}
+
+}  // namespace
+
+extern "C" int pcnn_conv_wgrad(pcnn_ctx *ctx, const void *x_bf16, const void *dy_bf16, float *dw_f32, int N, int H, int W, int C,
+                               int K, int R, int S, int row_pitch, int image_rows) {
+    return conv_wgrad("pcnn_conv_wgrad", ctx, x_bf16, dy_bf16, dw_f32, N, H, W, C, K, R, S, 1, row_pitch, image_rows);
+}
+
+extern "C" int pcnn_conv_wgrad_strided(pcnn_ctx *ctx, const void *x_bf16, const void *dy_bf16, float *dw_f32, int N, int H, int W, int C,
+                                       int K, int R, int S, int stride, int row_pitch, int image_rows) {
+    return conv_wgrad("pcnn_conv_wgrad_strided", ctx, x_bf16, dy_bf16, dw_f32, N, H, W, C, K, R, S, stride, row_pitch, image_rows);
+}
+
+extern "C" int pcnn_conv_dgrad(pcnn_ctx *ctx, const void *dy_bf16, const float *filt_f32_dev, void *dx_bf16, int N, int H, int W,
+                               int C, int K, int R, int S, int row_pitch, int image_rows) {
+    return conv_dgrad("pcnn_conv_dgrad", ctx, dy_bf16, filt_f32_dev, dx_bf16, N, H, W, C, K, R, S, 1, row_pitch, image_rows);
+}
+
+extern "C" int pcnn_conv_dgrad_strided(pcnn_ctx *ctx, const void *dy_bf16, const float *filt_f32_dev, void *dx_bf16, int N, int H, int W,
+                                       int C, int K, int R, int S, int stride, int row_pitch, int image_rows) {
+    return conv_dgrad("pcnn_conv_dgrad_strided", ctx, dy_bf16, filt_f32_dev, dx_bf16, N, H, W, C, K, R, S, stride, row_pitch, image_rows);
 }
 
 extern "C" int pcnn_conv_bwd_select(pcnn_ctx *ctx, int path) {
@@ -351,15 +382,21 @@ extern "C" int pcnn_crop_nhwc_bf16(pcnn_ctx *ctx, const void *src_bf16, void *ds
 // out[0] = weight gradient on the tensor cores (0/1), out[1..3] = its dy rows per tile, pixels per tile, stages;
 // out[4] = input gradient on the tensor cores (0/1), out[5..8] = its column strips, output pixels per lane quarter,
 // TMEM slot groups in flight, stages.  Pointer alignment and row pitch are assumed to qualify (16 bytes, multiple of 8).
-extern "C" int pcnn_conv_bwd_plan_info(int N, int H, int W, int C, int K, int R, int S, int *out9) {
+// The _strided query takes the window step (1..4); its out9[6] counts dx columns per lane quarter (stride x dy pixels).
+extern "C" int pcnn_conv_bwd_plan_info_strided(int N, int H, int W, int C, int K, int R, int S, int stride, int *out9) {
     PCNN_REQUIRE(out9 && N > 0 && H >= R && W >= S && C > 0 && K > 0 && R > 0 && S > 0, PCNN_ERR_ARG, "pcnn_conv_bwd_plan_info: bad argument");
+    PCNN_REQUIRE(stride >= 1 && stride <= 4, PCNN_ERR_ARG, "pcnn_conv_bwd_plan_info_strided: stride %d outside 1..4", stride);
     for (int i = 0; i < 9; ++i) out9[i] = 0;
     const void *aligned = reinterpret_cast<const void *>((uintptr_t)256);
     const int Kp = (K + 63) / 64 * 64;          // filter counts are zero-padded to a multiple of 64 (pcnn_conv_wgrad / dgrad)
-    if (pcnn_conv_wgrad_rows_ok(N, H, W, C, Kp, R, S, 8, aligned, aligned)) pcnn_conv_wgrad_rows_info(H, W, C, Kp, R, S, out9);
-    if (pcnn_conv_dgrad_rows_ok(N, H, W, C, Kp, R, S, aligned)) {
+    if (pcnn_conv_wgrad_rows_ok(N, H, W, C, Kp, R, S, stride, 8, aligned, aligned)) pcnn_conv_wgrad_rows_info(H, W, C, Kp, R, S, stride, out9);
+    if (pcnn_conv_dgrad_rows_ok(N, H, W, C, Kp, R, S, stride, aligned)) {
         out9[4] = 1;
-        pcnn_conv_dgrad_rows_info(H, W, C, Kp, R, S, out9 + 5);
+        pcnn_conv_dgrad_rows_info(H, W, C, Kp, R, S, stride, out9 + 5);
     }
     return PCNN_OK;
+}
+
+extern "C" int pcnn_conv_bwd_plan_info(int N, int H, int W, int C, int K, int R, int S, int *out9) {
+    return pcnn_conv_bwd_plan_info_strided(N, H, W, C, K, R, S, 1, out9);
 }

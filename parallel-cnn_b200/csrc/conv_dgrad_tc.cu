@@ -1,6 +1,7 @@
 // parallel-cnn_b200/csrc/conv_dgrad_tc.cu -- input gradient of the NHWC bf16 convolution (64 filters), row-streaming formulation.
 //
 //     dx[n][h][w][c] = sum_{k,r,s} dy[n][h-r][w-s][k] * f[k][r][s][c]
+//     (window step st: the sum runs over (h-r) % st == 0, (w-s) % st == 0 with dy[n][(h-r)/st][(w-s)/st][k])
 //
 // Access pattern first: a first version put 128 dy ROWS of one pixel column on the TMEM lanes (col2im folded into the TMEM
 // column offset); its TMA boxes gathered 128-byte pieces of 128 different rows, and a TMA pipeline with that pattern tops
@@ -18,6 +19,10 @@
 //   * Flow control is per group of 8 slots (tcgen05.commit -> tfull, epilogue -> tempty), NG groups in flight.
 //   * A CTA's share starts mid-image in general: the R-1 rows above it are replayed with filter variants that keep only the
 //     contributions landing inside the share (0.5 % extra reads at config 5).
+//   * Window step st > 1 (template parameter ST): the walk still covers every dx row; dy row h/st enters the ring at the slot of
+//     dx row h when h % st == 0.  A lane holds one dy pixel and owns the st dx columns (pixel + M - 1) * st + phi, M = ceil(S/st),
+//     phi < st: each is a sum over m of column (phi + m*st, c) of the lane m below it, so the boxes overlap by M - 1 pixels.
+//     Rows and columns no tap reaches come out as zeros.
 // TMEM addressing: the accumulator window of a tcgen05.mma must start on a multiple of 4 columns (an arbitrary column faults
 // with "misaligned address" on B200), hence SCP = 4*ceil(S*C/4) columns per slot.
 // Issue budget (pcnn_measure_mma_rate): one tcgen05.mma of N <= 112 occupies the issue/tensor path ~56-70 clk whatever its
@@ -39,7 +44,7 @@ constexpr int D2_SMEM_BUDGET = 200 * 1024;
 
 struct Dgrad2Params {
     int n_img, H, W, P, Q;
-    int nstrips, strip_w, oq, bp;        // strips per row, output columns per strip / per lane quarter, pixels per TMA box
+    int nstrips, strip_w, oq, bp;        // strips per row, output columns per strip, dy pixels per lane quarter / per TMA box
     int ng, ring, stages;                // slot groups in flight, ring slots (8 * ng), smem stages
     int KH;                              // channels / 64: a TMA box holds 64 channels (one 128-byte swizzle row per pixel)
     long long T;                         // n_img * H output rows in walk order
@@ -78,10 +83,11 @@ struct RowWalk {
     }
 };
 
-template <int R, int S, int C, int KHC>
+template <int R, int S, int C, int KHC, int ST>
 __global__ void __launch_bounds__(D2_THREADS, 1)
 k_conv_tc_dgrad_rows(const __grid_constant__ CUtensorMap map_dy, const __grid_constant__ CUtensorMap map_b, const Dgrad2Params p) {
     constexpr int SC = S * C, SCP = (SC + 3) / 4 * 4, NW = (R * SCP + 15) / 16 * 16;
+    constexpr int M = (S + ST - 1) / ST;                               // dy pixels that reach one dx column
     extern __shared__ unsigned char smem_dyn[];
     unsigned char *base = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
     constexpr int BMAT = NW * 128;
@@ -139,15 +145,15 @@ k_conv_tc_dgrad_rows(const __grid_constant__ CUtensorMap map_dy, const __grid_co
             int n = n_first, h = h_first - warm;
             const long long nrows = nel + warm;
             for (long long i = 0; i < nrows; ++i) {
-                if (h < p.P) {
+                if (h % ST == 0 && h / ST < p.P) {     // dy row h / st enters at dx row h
                     bar_wait_relaxed(&B.empty[stage], ph ^ 1u, 32);
                     bar_expect_tx(&B.full[stage], (unsigned)(KH * 4 * p.bp * 128));
                     unsigned char *a = astage + (size_t)stage * STAGE;
-                    const int row = n * p.P + h;
+                    const int row = n * p.P + h / ST;
                     for (int kh = 0; kh < KH; ++kh)
 #pragma unroll
                         for (int g = 0; g < 4; ++g)      // pixels left of the image / right of its last dy pixel arrive as zeros
-                            tma_load_3d(a + kh * D2_HALF_BYTES + g * 4096, &map_dy, kh * 64, w_strip + g * p.oq - (S - 1), row, &B.full[stage]);
+                            tma_load_3d(a + kh * D2_HALF_BYTES + g * 4096, &map_dy, kh * 64, w_strip / ST + g * p.oq - (M - 1), row, &B.full[stage]);
                     if (++stage == NST) { stage = 0; ph ^= 1u; }
                 }
                 if (++h == p.H) { h = 0; ++n; }
@@ -173,7 +179,7 @@ k_conv_tc_dgrad_rows(const __grid_constant__ CUtensorMap map_dy, const __grid_co
                     bar_wait(&B.tempty[rg], (unsigned)(((G + 1) / NG - 1) & 1));
                     tc_fence_after();
                 }
-                if (h < p.P) {
+                if (h % ST == 0 && h / ST < p.P) {
                     bar_wait(&B.full[stage], ph);
                     tc_fence_after();
                     uint64_t ad = adesc0 + (uint64_t)((uint32_t)stage * ((uint32_t)STAGE >> 4));
@@ -203,9 +209,9 @@ k_conv_tc_dgrad_rows(const __grid_constant__ CUtensorMap map_dy, const __grid_co
         // ===== epilogue: drain completed rows, sum over s across lanes, store, re-zero =====
         const int quarter = warp & 3;
         const uint32_t tq = tmem + ((uint32_t)(quarter * 32) << 16);
-        const int w_q0 = w_strip + quarter * p.oq;
-        int nvalid = w_end - w_q0;                           // output pixels of this quarter
-        if (nvalid > p.oq) nvalid = p.oq;
+        const int w_q0 = w_strip + quarter * p.oq * ST;
+        int nvalid = w_end - w_q0;                           // output columns of this quarter
+        if (nvalid > p.oq * ST) nvalid = p.oq * ST;
         int n = n_first, h = h_first, pos = 0;
         const int ngroups = (int)((nel + D2_GROUP - 1) / D2_GROUP);
         for (int G = 0; G < ngroups; ++G) {
@@ -224,25 +230,32 @@ k_conv_tc_dgrad_rows(const __grid_constant__ CUtensorMap map_dy, const __grid_co
                     for (int j = 0; j < SCP; j += 4) tc_ld_32x4(tq + (uint32_t)((RING + pos) * SCP) + j, u[j], u[j + 1], u[j + 2], u[j + 3]);
                 }
                 tc_wait_ld();
-                float o[C];
+                float o[ST * C];
 #pragma unroll
-                for (int c = 0; c < C; ++c) o[c] = 0.0f;
+                for (int c = 0; c < ST * C; ++c) o[c] = 0.0f;
 #pragma unroll
-                for (int s = 0; s < S; ++s) {
+                for (int m = 0; m < M; ++m) {
 #pragma unroll
-                    for (int c = 0; c < C; ++c) {
-                        float x = __uint_as_float(v[s * C + c]);
-                        if (tail) x += __uint_as_float(u[s * C + c]);
-                        // lane l holds dy pixel (first + l); output pixel l of the quarter needs dy pixel l + (S-1) - s
-                        if (S - 1 - s > 0) x = __shfl_down_sync(0xFFFFFFFFu, x, S - 1 - s);
-                        o[c] += x;
+                    for (int phi = 0; phi < ST; ++phi) {
+                        const int s = phi + m * ST;
+                        if (s >= S) continue;
+#pragma unroll
+                        for (int c = 0; c < C; ++c) {
+                            float x = __uint_as_float(v[s * C + c]);
+                            if (tail) x += __uint_as_float(u[s * C + c]);
+                            // lane l holds dy pixel (first + l); its dx columns (first + l + M-1) * st + phi need dy pixel l + (M-1) - m
+                            if (M - 1 - m > 0) x = __shfl_down_sync(0xFFFFFFFFu, x, M - 1 - m);
+                            o[phi * C + c] += x;
+                        }
                     }
                 }
-                if (lane < nvalid) {
-                    __nv_bfloat16 *dst = p.dx + ((long long)n * p.dx_image_rows + h) * p.dx_pitch + (long long)(w_q0 + lane) * C;
+                __nv_bfloat16 *dst = p.dx + ((long long)n * p.dx_image_rows + h) * p.dx_pitch + (long long)(w_q0 + lane * ST) * C;
 #pragma unroll
-                    for (int c = 0; c < C; ++c) dst[c] = __float2bfloat16_rn(o[c]);
-                }
+                for (int phi = 0; phi < ST; ++phi)
+                    if (lane * ST + phi < nvalid) {
+#pragma unroll
+                        for (int c = 0; c < C; ++c) dst[phi * C + c] = __float2bfloat16_rn(o[phi * C + c]);
+                    }
 #pragma unroll
                 for (int j = 0; j < SCP; j += 4) tc_st_zero_32x4(c0 + j);
                 if (tail) {
@@ -277,59 +290,83 @@ Geometry geometry(int R, int S, int C) {
     return g;
 }
 
-template <int R, int S, int C, int KHC>
+template <int R, int S, int C, int KHC, int ST>
 int launch_rows_k(pcnn_ctx *ctx, const CUtensorMap &map_dy, const CUtensorMap &map_b, const Dgrad2Params &p, int grid, size_t smem) {
     static bool configured[64] = {};        // function attributes are per device
     if (!configured[ctx->device & 63]) {
-        PCNN_CUDA(cudaFuncSetAttribute(k_conv_tc_dgrad_rows<R, S, C, KHC>, cudaFuncAttributeMaxDynamicSharedMemorySize, D2_SMEM_BUDGET + 2048));
+        PCNN_CUDA(cudaFuncSetAttribute(k_conv_tc_dgrad_rows<R, S, C, KHC, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, D2_SMEM_BUDGET + 2048));
         configured[ctx->device & 63] = true;
     }
-    k_conv_tc_dgrad_rows<R, S, C, KHC><<<grid, D2_THREADS, smem, ctx->stream>>>(map_dy, map_b, p);
+    k_conv_tc_dgrad_rows<R, S, C, KHC, ST><<<grid, D2_THREADS, smem, ctx->stream>>>(map_dy, map_b, p);
     PCNN_CHECK_LAUNCH(ctx);
     return PCNN_OK;
 }
-template <int R, int S, int C>
+template <int R, int S, int C, int ST>
 int launch_rows(pcnn_ctx *ctx, const CUtensorMap &map_dy, const CUtensorMap &map_b, const Dgrad2Params &p, int grid, size_t smem) {
-    return p.KH == 1 ? launch_rows_k<R, S, C, 1>(ctx, map_dy, map_b, p, grid, smem) : launch_rows_k<R, S, C, 0>(ctx, map_dy, map_b, p, grid, smem);
+    return p.KH == 1 ? launch_rows_k<R, S, C, 1, ST>(ctx, map_dy, map_b, p, grid, smem) : launch_rows_k<R, S, C, 0, ST>(ctx, map_dy, map_b, p, grid, smem);
+}
+
+// the built (R, S, C, stride) combinations, in one place for the predicate and the dispatch: every 3x3 (C in {1,2,3,4,8}), 5x5
+// (C in {1,3}) and 7x7 (C = 1) kernel at strides 1 and 2; 3x3 with C in {1,2,3} at stride 3; 3x3x3 and 5x5x1 at stride 4
+#define PCNN_DGRAD_ROWS_KERNELS(X)                                                                                               \
+    X(3, 3, 3, 1) X(3, 3, 1, 1) X(3, 3, 4, 1) X(5, 5, 1, 1) X(3, 3, 2, 1) X(3, 3, 8, 1) X(5, 5, 3, 1) X(7, 7, 1, 1)            \
+    X(3, 3, 3, 2) X(3, 3, 1, 2) X(3, 3, 4, 2) X(5, 5, 1, 2) X(3, 3, 2, 2) X(3, 3, 8, 2) X(5, 5, 3, 2) X(7, 7, 1, 2)            \
+    X(3, 3, 1, 3) X(3, 3, 2, 3) X(3, 3, 3, 3)                                                                                   \
+    X(3, 3, 3, 4) X(5, 5, 1, 4)
+
+bool instantiated(int R, int S, int C, int st) {
+#define X(r, s, c, t) if (R == r && S == s && C == c && st == t) return true;
+    PCNN_DGRAD_ROWS_KERNELS(X)
+#undef X
+    return false;
+}
+
+// column strips of a multiple of st dx columns; a lane quarter takes oq dy pixels = oq * st dx columns, at most 32 - (M - 1)
+// pixels (its box holds oq + M - 1 <= 32 pixels)
+struct Strips { int nstrips, strip_w, oq; };
+Strips strips(int W, int S, int st) {
+    Strips t;
+    const int oq_max = 32 - ((S + st - 1) / st - 1);
+    t.nstrips = (W + 4 * oq_max * st - 1) / (4 * oq_max * st);
+    t.strip_w = ((W + t.nstrips - 1) / t.nstrips + st - 1) / st * st;
+    t.oq = (t.strip_w / st + 3) / 4;
+    return t;
 }
 
 }  // namespace
 
-bool pcnn_conv_dgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, const void *dy) {
+bool pcnn_conv_dgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, int stride, const void *dy) {
     if (K % 64 || K > 256 || ((uintptr_t)dy & 15) || N <= 0 || H < R || W < S) return false;
-    const bool inst = (R == 3 && S == 3 && (C == 1 || C == 2 || C == 3 || C == 4 || C == 8)) || (R == 5 && S == 5 && (C == 1 || C == 3)) ||
-                      (R == 7 && S == 7 && C == 1);
-    if (!inst) return false;
+    if (!instantiated(R, S, C, stride)) return false;
     const Geometry g = geometry(R, S, C);
     return g.ng >= 2 && g.nw <= 256 && S <= 16;
 }
 
 // host-side tiling of the row-streaming input gradient, for pcnn_conv_bwd_plan_info (no GPU needed)
-void pcnn_conv_dgrad_rows_info(int H, int W, int C, int K, int R, int S, int *out4) {
+void pcnn_conv_dgrad_rows_info(int H, int W, int C, int K, int R, int S, int stride, int *out4) {
     const Geometry g = geometry(R, S, C);
-    const int oq_max = 32 - (S - 1);
-    const int nstrips = (W + 4 * oq_max - 1) / (4 * oq_max), strip_w = (W + nstrips - 1) / nstrips;
+    const Strips t = strips(W, S, stride);
     const size_t stage_bytes = (size_t)(K / 64) * D2_HALF_BYTES;
     const size_t fixed = (size_t)R * (K / 64) * g.nw * 128 + sizeof(Dgrad2Ctl) + 1024;
     int st = stage_bytes ? (int)(((size_t)D2_SMEM_BUDGET - fixed) / stage_bytes) : 0;
-    out4[0] = nstrips; out4[1] = (strip_w + 3) / 4; out4[2] = g.ng; out4[3] = st > D2_MAX_STAGES ? D2_MAX_STAGES : st;
+    out4[0] = t.nstrips; out4[1] = t.oq * stride; out4[2] = g.ng; out4[3] = st > D2_MAX_STAGES ? D2_MAX_STAGES : st;
     (void)H;
 }
 
 // dy_channels: as for pcnn_conv_wgrad_rows (filters dy really holds; the TMA zero-fills the rest of a 64-channel box)
 int pcnn_conv_dgrad_rows(pcnn_ctx *ctx, const void *dy_bf16, const float *filt_f32_dev, void *dx_bf16, int N, int H, int W, int C, int K,
-                         int R, int S, int row_pitch, int image_rows, int dy_channels) {
+                         int R, int S, int stride, int row_pitch, int image_rows, int dy_channels) {
     const uint64_t KD = dy_channels > 0 ? (uint64_t)dy_channels : (uint64_t)K;
     pcnn_device_guard guard(ctx->device);
     const Geometry g = geometry(R, S, C);
     Dgrad2Params p;
     memset(&p, 0, sizeof(p));
-    p.n_img = N; p.H = H; p.W = W; p.P = H - R + 1; p.Q = W - S + 1;
-    const int oq_max = 32 - (S - 1);
-    p.nstrips = (W + 4 * oq_max - 1) / (4 * oq_max);
-    p.strip_w = (W + p.nstrips - 1) / p.nstrips;
-    p.oq = (p.strip_w + 3) / 4;
-    p.bp = p.oq + S - 1;
+    p.n_img = N; p.H = H; p.W = W; p.P = (H - R) / stride + 1; p.Q = (W - S) / stride + 1;
+    const Strips t = strips(W, S, stride);
+    p.nstrips = t.nstrips;
+    p.strip_w = t.strip_w;
+    p.oq = t.oq;
+    p.bp = p.oq + (S + stride - 1) / stride - 1;
     p.ng = g.ng;
     p.ring = D2_GROUP * g.ng;
     p.T = (long long)N * H;
@@ -367,14 +404,9 @@ int pcnn_conv_dgrad_rows(pcnn_ctx *ctx, const void *dy_bf16, const float *filt_f
     // every CTA needs at least one row of its strip; more CTAs than rows would leave empty shares (handled, but pointless)
     long long want = p.T * p.nstrips;
     const int grid = (int)(want < ctx->sm_count ? want : ctx->sm_count);
-    if (R == 3 && S == 3 && C == 3) return launch_rows<3, 3, 3>(ctx, map_dy, map_b, p, grid, smem);
-    if (R == 3 && S == 3 && C == 1) return launch_rows<3, 3, 1>(ctx, map_dy, map_b, p, grid, smem);
-    if (R == 3 && S == 3 && C == 4) return launch_rows<3, 3, 4>(ctx, map_dy, map_b, p, grid, smem);
-    if (R == 5 && S == 5 && C == 1) return launch_rows<5, 5, 1>(ctx, map_dy, map_b, p, grid, smem);
-    if (R == 3 && S == 3 && C == 2) return launch_rows<3, 3, 2>(ctx, map_dy, map_b, p, grid, smem);
-    if (R == 3 && S == 3 && C == 8) return launch_rows<3, 3, 8>(ctx, map_dy, map_b, p, grid, smem);
-    if (R == 5 && S == 5 && C == 3) return launch_rows<5, 5, 3>(ctx, map_dy, map_b, p, grid, smem);
-    if (R == 7 && S == 7 && C == 1) return launch_rows<7, 7, 1>(ctx, map_dy, map_b, p, grid, smem);
-    pcnn_set_error("pcnn_conv_dgrad: no row-streaming instantiation for R = %d, S = %d, C = %d", R, S, C);
+#define X(r, s, c, t) if (R == r && S == s && C == c && stride == t) return launch_rows<r, s, c, t>(ctx, map_dy, map_b, p, grid, smem);
+    PCNN_DGRAD_ROWS_KERNELS(X)
+#undef X
+    pcnn_set_error("pcnn_conv_dgrad: no row-streaming instantiation for R = %d, S = %d, C = %d, stride %d", R, S, C, stride);
     return PCNN_ERR_ARG;
 }

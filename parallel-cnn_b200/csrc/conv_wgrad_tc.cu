@@ -1,6 +1,6 @@
 // parallel-cnn_b200/csrc/conv_wgrad_tc.cu -- weight gradient of the NHWC bf16 convolution (64 filters) on the tcgen05 tensor cores.
 //
-//     dw[k][r][s][c] = sum_{n,p,q} dy[n][p][q][k] * x[n][p+r][q+s][c]           [ref: layer.h:371-395 bp_weight_c1, without /576]
+//     dw[k][r][s][c] = sum_{n,p,q} dy[n][p][q][k] * x[n][p*st+r][q*st+s][c]     [ref: layer.h:371-395 bp_weight_c1, without /576]
 //
 // SURVEY.md x3 / BASELINE.json config 5: dy [N,222,222,64] is 95 % of the 6.6 MB/image this pass moves and the pass is
 // HBM-bound (SURVEY.md 8d), so: dy crosses HBM -> shared memory once by TMA and is consumed there by tcgen05.mma.
@@ -10,9 +10,11 @@
 //   * The other operand is the Hankel matrix of the x rows, A[(rho, s, c)][pixel q] = x[p0 + rho][(q + s) * C + c] for the
 //     RB + R - 1 input rows a block of RB dy rows touches (54 of M = 64 rows at config 5); eight warps build it in shared
 //     memory from the x row segments (x is 5 % of the traffic; the 9x expansion never leaves the SM).
+//     Window step st > 1: A[(rho, s, c)][q] = x[p0*st + rho][(q*st + s) * C + c] over the (RB-1)*st + R x rows of the block
+//     (the builders gather with a stride of st*C elements); the dy tiles and the MMAs do not change.
 //     (More than 64 filters: K/64 boxes per tile, the accumulator columns become (filter group, row, filter), K <= 256.)
 //   * D[(rho, s, c)][(row, k)] accumulates in ONE 64 x 256 TMEM accumulator for the whole kernel; the entries with
-//     rho - row = r in [0, R) are the gradient, the others are discarded.  At the end each CTA folds the RB row blocks,
+//     rho - row*st = r in [0, R) are the gradient, the others are discarded.  At the end each CTA folds the RB row blocks,
 //     writes one 1,728-float partial, and a second kernel adds the partials in a fixed order (deterministic, no atomics).
 // Why this shape: one tcgen05.mma costs the issuing thread and the tensor path ~56-70 clk for any N <= 112 and N/2 clk
 // above (pcnn_measure_mma_rate), and a first version with one dy row per tile (dy as the M = 64 operand, N = 32) was bound
@@ -61,15 +63,16 @@ __device__ __forceinline__ void sts_v4(uint32_t saddr, uint4 v) {
 }
 
 // bytes of x row segment `chunk` that exist in the row (a multiple of 16; 0 when the chunk starts past the row)
+template <int ST>
 __device__ __forceinline__ int xseg_copy_bytes(const Wgrad2Params &p, int chunk) {
-    const int start = chunk * p.PC * p.C * 2;
+    const int start = chunk * p.PC * ST * p.C * 2;
     int avail = p.xrow_bytes - start;
     if (avail < 0) avail = 0;
     return avail < p.xseg_bytes ? avail : p.xseg_bytes;
 }
 
-// CT = compile-time input-channel count (the gather stride of the Hankel builder), 0 = run-time
-template <int CT>
+// CT = compile-time input-channel count (the gather stride of the Hankel builder), 0 = run-time; ST = window step
+template <int CT, int ST>
 __global__ void __launch_bounds__(W2_THREADS, 1)
 k_conv_tc_wgrad_rows(const __grid_constant__ CUtensorMap map_dy, const Wgrad2Params p) {
     const int C = CT > 0 ? CT : p.C;
@@ -113,8 +116,8 @@ k_conv_tc_wgrad_rows(const __grid_constant__ CUtensorMap map_dy, const Wgrad2Par
             for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
                 const int n = tile / tiles_per_img, rem = tile % tiles_per_img, pb = rem / p.n_ch, ch = rem % p.n_ch;
                 const int p0 = pb * p.RB;
-                const int xb = xseg_copy_bytes(p, ch);
-                int nx = p.H - p0;                        // x rows p0 .. p0 + NXR - 1 that exist
+                const int xb = xseg_copy_bytes<ST>(p, ch);
+                int nx = p.H - p0 * ST;                   // x rows p0*st .. p0*st + NXR - 1 that exist
                 if (nx > p.NXR) nx = p.NXR;
                 bar_wait_relaxed(&S.empty[stage], ph ^ 1u, 32);
                 bar_expect_tx(&S.full[stage], (unsigned)(dy_bytes + nx * xb));
@@ -123,7 +126,7 @@ k_conv_tc_wgrad_rows(const __grid_constant__ CUtensorMap map_dy, const Wgrad2Par
                 if (xb > 0)
                     for (int r = 0; r < nx; ++r)
                         tma_load_1d(X + (size_t)stage * x_bytes + (size_t)r * p.xseg_stride,
-                                    p.x + ((long long)n * p.x_image_rows + p0 + r) * p.x_pitch + (long long)ch * p.PC * C, (unsigned)xb,
+                                    p.x + ((long long)n * p.x_image_rows + p0 * ST + r) * p.x_pitch + (long long)ch * p.PC * ST * C, (unsigned)xb,
                                     &S.full[stage]);
                 if (++stage == NST) { stage = 0; ph ^= 1u; }
             }
@@ -169,7 +172,7 @@ k_conv_tc_wgrad_rows(const __grid_constant__ CUtensorMap map_dy, const Wgrad2Par
                 const int n8 = L / (p.KO * 8), rem = L % (p.KO * 8), kk = rem >> 3, nl = rem & 7, n = n8 * 8 + nl;
                 if (n < p.nreal) {
                     const int rho = n / p.SC, j = n % p.SC;
-                    e0s[i] = kk * 8 * C + j;                 // element of the x segment feeding pixel 8*kk of the tile
+                    e0s[i] = kk * 8 * ST * C + j;            // element of the x segment feeding pixel 8*kk of the tile
                     src_off[i] = rho * p.xseg_stride + e0s[i] * 2;
                     dst_off[i] = n8 * SBO + kk * 128 + nl * 16;
                 }
@@ -186,17 +189,17 @@ k_conv_tc_wgrad_rows(const __grid_constant__ CUtensorMap map_dy, const Wgrad2Par
             for (int i = 0; i < W2_ITEMS; ++i) {             // all gathers in flight before the first use
                 const uint32_t src = xs + (uint32_t)(src_off[i] >= 0 ? src_off[i] : 0);
 #pragma unroll
-                for (int u = 0; u < 8; ++u) e[i][u] = lds_u16(src + (uint32_t)(u * C * 2));
+                for (int u = 0; u < 8; ++u) e[i][u] = lds_u16(src + (uint32_t)(u * ST * C * 2));
             }
             int lim0 = 0;
-            if (p.guard) lim0 = p.W * C - ((tile % tiles_per_img) % p.n_ch) * p.PC * C;   // row elements at or after the segment start
+            if (p.guard) lim0 = p.W * C - ((tile % tiles_per_img) % p.n_ch) * p.PC * ST * C;   // row elements at or after the segment start
 #pragma unroll
             for (int i = 0; i < W2_ITEMS; ++i) {
                 if (src_off[i] >= 0) {
                     if (p.guard) {
 #pragma unroll
                         for (int u = 0; u < 8; ++u)
-                            if (e0s[i] + u * C >= lim0) e[i][u] = 0;
+                            if (e0s[i] + u * ST * C >= lim0) e[i][u] = 0;
                     }
                     uint4 o;
                     o.x = e[i][0] | ((uint32_t)e[i][1] << 16); o.y = e[i][2] | ((uint32_t)e[i][3] << 16);
@@ -231,13 +234,13 @@ k_conv_tc_wgrad_rows(const __grid_constant__ CUtensorMap map_dy, const Wgrad2Par
     tc_fence_before();
     __syncthreads();
     {
-        // dw[k][r][j] = sum over row blocks rb of D[(rb + r) * SC + j][rb * 64 + k]
+        // dw[k][r][j] = sum over row blocks rb of D[(rb * st + r) * SC + j][rb * 64 + k]
         const int K = p.KH * 64;
         float *dst = p.slots + (size_t)blockIdx.x * K * p.nout;
         for (int o = threadIdx.x; o < K * p.nout; o += W2_THREADS) {
             const int k = o / p.nout, rj = o % p.nout, r = rj / p.SC, j = rj % p.SC, kh = k >> 6, kl = k & 63;
             float s = 0.0f;
-            for (int rb = 0; rb < p.RB; ++rb) s += dump[((rb + r) * p.SC + j) * W2_DUMP_STRIDE + (kh * p.RB + rb) * 64 + kl];
+            for (int rb = 0; rb < p.RB; ++rb) s += dump[((rb * ST + r) * p.SC + j) * W2_DUMP_STRIDE + (kh * p.RB + rb) * 64 + kl];
             dst[o] = s;
         }
     }
@@ -267,19 +270,21 @@ struct Plan { int RB, PC, stages; size_t stage_bytes, smem; bool ok; };
 // Tile shape: dy rows per tile RB (N = RB * 64) and pixels per tile PC.  Measured at config 5 (profiles/r01_README.md): what
 // matters is that the tiles cover the [P x Q] plane with little padding (PC = 112 covers Q = 222 in two chunks: 139-147 us;
 // PC = 80 in three: 149-244 us) and that at least three stages fit; RB = 3 (139 us) ~ RB = 2 (141 us) < RB = 4 (147 us, two
-// stages).
-Plan plan_for(int P, int Q, int C, int R, int S, int KH) {
+// stages).  Window step st: a block of RB dy rows reads (RB - 1) * st + R x rows, a chunk of PC pixels ((PC - 1) * st + S) * C
+// elements of each.
+Plan plan_for(int P, int Q, int C, int R, int S, int KH, int st) {
     Plan pl;
     memset(&pl, 0, sizeof(pl));
     const int SC = S * C;
     double best = -1.0;
     for (int RB = 4; RB >= 1; --RB) {
-        if ((RB + R - 1) * SC > 64 || RB * KH * 64 > 256) continue;
+        const int NXR = (RB - 1) * st + R;
+        if (NXR * SC > 64 || RB * KH * 64 > 256) continue;
         for (int PC = 128; PC >= 32; PC -= 16) {
-            const int units = (((RB + R - 1) * SC + 7) / 8) * 8 * (PC / 8);
+            const int units = ((NXR * SC + 7) / 8) * 8 * (PC / 8);
             if (units > W2_ITEMS * 32 * W2_BUILD_WARPS) continue;
-            const size_t xseg = (size_t)(((PC + S) * C * 2 + 127) / 128 * 128);
-            const size_t stage = (size_t)KH * RB * PC * 128 + (size_t)64 * PC * 2 + (size_t)(RB + R - 1) * xseg;
+            const size_t xseg = (size_t)((((PC - 1) * st + S + 1) * C * 2 + 127) / 128 * 128);
+            const size_t stage = (size_t)KH * RB * PC * 128 + (size_t)64 * PC * 2 + (size_t)NXR * xseg;
             int st = (int)(((size_t)W2_SMEM_BUDGET - sizeof(Wgrad2Ctl) - 1024) / stage);
             if (st > W2_MAX_STAGES) st = W2_MAX_STAGES;
             if (st < 2) continue;
@@ -297,50 +302,56 @@ Plan plan_for(int P, int Q, int C, int R, int S, int KH) {
     return pl;
 }
 
-template <int CT>
+template <int CT, int ST>
 int launch_rows(pcnn_ctx *ctx, const CUtensorMap &map_dy, const Wgrad2Params &p, int grid, size_t smem) {
     static bool configured[64] = {};        // function attributes are per device
     if (!configured[ctx->device & 63]) {
-        PCNN_CUDA(cudaFuncSetAttribute(k_conv_tc_wgrad_rows<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, W2_SMEM_BUDGET + 2048));
+        PCNN_CUDA(cudaFuncSetAttribute(k_conv_tc_wgrad_rows<CT, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, W2_SMEM_BUDGET + 2048));
         configured[ctx->device & 63] = true;
     }
-    k_conv_tc_wgrad_rows<CT><<<grid, W2_THREADS, smem, ctx->stream>>>(map_dy, p);
+    k_conv_tc_wgrad_rows<CT, ST><<<grid, W2_THREADS, smem, ctx->stream>>>(map_dy, p);
     PCNN_CHECK_LAUNCH(ctx);
     return PCNN_OK;
+}
+template <int ST>
+int launch_rows_c(pcnn_ctx *ctx, const CUtensorMap &map_dy, const Wgrad2Params &p, int grid, size_t smem) {
+    return p.C == 3 ? launch_rows<3, ST>(ctx, map_dy, p, grid, smem) : p.C == 1 ? launch_rows<1, ST>(ctx, map_dy, p, grid, smem)
+         : p.C == 4 ? launch_rows<4, ST>(ctx, map_dy, p, grid, smem) : launch_rows<0, ST>(ctx, map_dy, p, grid, smem);
 }
 
 }  // namespace
 
-bool pcnn_conv_wgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, int row_pitch, const void *x, const void *dy) {
+bool pcnn_conv_wgrad_rows_ok(int N, int H, int W, int C, int K, int R, int S, int stride, int row_pitch, const void *x, const void *dy) {
     if (K % 64 || K > 256 || ((uintptr_t)dy & 15) || ((uintptr_t)x & 15) || row_pitch % 8 || N <= 0 || H < R || W < S) return false;
-    return plan_for(H - R + 1, W - S + 1, C, R, S, K / 64).ok;
+    if (stride < 1 || stride > 4) return false;
+    return plan_for((H - R) / stride + 1, (W - S) / stride + 1, C, R, S, K / 64, stride).ok;
 }
 
 // host-side tile choice of the weight gradient, for pcnn_conv_bwd_plan_info (no GPU needed)
-void pcnn_conv_wgrad_rows_info(int H, int W, int C, int K, int R, int S, int *out4) {
-    const Plan pl = plan_for(H - R + 1, W - S + 1, C, R, S, K / 64);
+void pcnn_conv_wgrad_rows_info(int H, int W, int C, int K, int R, int S, int stride, int *out4) {
+    const Plan pl = plan_for((H - R) / stride + 1, (W - S) / stride + 1, C, R, S, K / 64, stride);
     out4[0] = pl.ok ? 1 : 0; out4[1] = pl.RB; out4[2] = pl.PC; out4[3] = pl.stages;
 }
 
 // dy_channels: filters dy really holds per pixel (<= K, multiple of 8: 16-byte pixel pitch); the TMA boxes stay 64 channels
 // wide and the hardware fills channels dy_channels..63 of a box with zeros, so a 16- or 32-filter gradient needs no padded copy
 int pcnn_conv_wgrad_rows(pcnn_ctx *ctx, const void *x_bf16, const void *dy_bf16, float *dw_f32, int N, int H, int W, int C, int K,
-                         int R, int S, int row_pitch, int image_rows, int dy_channels) {
+                         int R, int S, int stride, int row_pitch, int image_rows, int dy_channels) {
     const uint64_t KD = dy_channels > 0 ? (uint64_t)dy_channels : (uint64_t)K;
     pcnn_device_guard g(ctx->device);
-    const int P = H - R + 1, Q = W - S + 1;
-    const Plan pl = plan_for(P, Q, C, R, S, K / 64);
+    const int P = (H - R) / stride + 1, Q = (W - S) / stride + 1;
+    const Plan pl = plan_for(P, Q, C, R, S, K / 64, stride);
     PCNN_REQUIRE(pl.ok, PCNN_ERR_ARG, "pcnn_conv_wgrad: shape does not fit the tensor-core kernel");
     Wgrad2Params p;
     memset(&p, 0, sizeof(p));
     p.n_img = N; p.H = H; p.P = P; p.Q = Q; p.W = W; p.C = C; p.R = R; p.SC = S * C;
-    p.RB = pl.RB; p.NXR = pl.RB + R - 1; p.PC = pl.PC; p.KO = pl.PC / 8; p.KH = K / 64;
+    p.RB = pl.RB; p.NXR = (pl.RB - 1) * stride + R; p.PC = pl.PC; p.KO = pl.PC / 8; p.KH = K / 64;
     p.nreal = p.NXR * p.SC; p.nout = R * p.SC;
     p.n_pb = (P + p.RB - 1) / p.RB; p.n_ch = (Q + p.PC - 1) / p.PC; p.stages = pl.stages;
     p.x_pitch = row_pitch > 0 ? row_pitch : W * C;
     p.x_image_rows = image_rows > 0 ? image_rows : H;
-    p.xseg_bytes = ((p.PC + S - 1) * C * 2 + 15) / 16 * 16;
-    p.xseg_stride = ((p.PC + S) * C * 2 + 127) / 128 * 128;
+    p.xseg_bytes = (((p.PC - 1) * stride + S) * C * 2 + 15) / 16 * 16;
+    p.xseg_stride = ((((p.PC - 1) * stride + S + 1) * C * 2 + 127) / 128 * 128);
     p.xrow_bytes = (W * C * 2 + 15) / 16 * 16;
     PCNN_REQUIRE((long long)p.xrow_bytes <= p.x_pitch * 2 && p.xseg_bytes <= p.xseg_stride, PCNN_ERR_ARG, "pcnn_conv_wgrad: row pitch");
     p.guard = (W * C * 2) % 16 != 0;
@@ -359,8 +370,8 @@ int pcnn_conv_wgrad_rows(pcnn_ctx *ctx, const void *x_bf16, const void *dy_bf16,
                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B)))
             return rc;
     }
-    rc = C == 3 ? launch_rows<3>(ctx, map_dy, p, grid, pl.smem) : C == 1 ? launch_rows<1>(ctx, map_dy, p, grid, pl.smem)
-       : C == 4 ? launch_rows<4>(ctx, map_dy, p, grid, pl.smem) : launch_rows<0>(ctx, map_dy, p, grid, pl.smem);
+    rc = stride == 1 ? launch_rows_c<1>(ctx, map_dy, p, grid, pl.smem) : stride == 2 ? launch_rows_c<2>(ctx, map_dy, p, grid, pl.smem)
+       : stride == 3 ? launch_rows_c<3>(ctx, map_dy, p, grid, pl.smem) : launch_rows_c<4>(ctx, map_dy, p, grid, pl.smem);
     if (rc) return rc;
     k_conv_tc_wgrad_rows_reduce<<<(nout + 31) / 32, 256, 0, ctx->stream>>>(p.slots, dw_f32, grid, nout);
     PCNN_CHECK_LAUNCH(ctx);

@@ -375,11 +375,21 @@ class Engine:
         """reference=True: the FMA-pipe reference kernels for every shape (explicit opt-in); False: tensor cores only"""
         self._call("pcnn_conv_bwd_select", 1 if reference else 0)
 
-    def conv_wgrad(self, x_bf16, dy_bf16, dw_f32, N, H, W, Cin, K, R, S, row_pitch=0, image_rows=0):
-        self._call("pcnn_conv_wgrad", _p(x_bf16), _p(dy_bf16), _p(dw_f32), N, H, W, Cin, K, R, S, int(row_pitch), int(image_rows))
+    def conv_wgrad(self, x_bf16, dy_bf16, dw_f32, N, H, W, Cin, K, R, S, row_pitch=0, image_rows=0, stride=1):
+        """weight gradient; stride > 1: the window step of a strided forward plan (dy [N][(H-R)//stride+1][(W-S)//stride+1][K])"""
+        if stride == 1:
+            self._call("pcnn_conv_wgrad", _p(x_bf16), _p(dy_bf16), _p(dw_f32), N, H, W, Cin, K, R, S, int(row_pitch), int(image_rows))
+        else:
+            self._call("pcnn_conv_wgrad_strided", _p(x_bf16), _p(dy_bf16), _p(dw_f32), N, H, W, Cin, K, R, S, int(stride), int(row_pitch),
+                       int(image_rows))
 
-    def conv_dgrad(self, dy_bf16, filt_f32, dx_bf16, N, H, W, Cin, K, R, S, row_pitch=0, image_rows=0):
-        self._call("pcnn_conv_dgrad", _p(dy_bf16), _p(filt_f32), _p(dx_bf16), N, H, W, Cin, K, R, S, int(row_pitch), int(image_rows))
+    def conv_dgrad(self, dy_bf16, filt_f32, dx_bf16, N, H, W, Cin, K, R, S, row_pitch=0, image_rows=0, stride=1):
+        """input gradient; stride as for conv_wgrad (every dx element is written, those no tap reaches as 0)"""
+        if stride == 1:
+            self._call("pcnn_conv_dgrad", _p(dy_bf16), _p(filt_f32), _p(dx_bf16), N, H, W, Cin, K, R, S, int(row_pitch), int(image_rows))
+        else:
+            self._call("pcnn_conv_dgrad_strided", _p(dy_bf16), _p(filt_f32), _p(dx_bf16), N, H, W, Cin, K, R, S, int(stride), int(row_pitch),
+                       int(image_rows))
 
     def pad_nhwc(self, src_bf16, dst_bf16, N, H, W, Cin, pad_h, pad_w, dst_row_pitch=0, dst_image_rows=0):
         self._call("pcnn_pad_nhwc_bf16", _p(src_bf16), _p(dst_bf16), N, H, W, Cin, int(pad_h), int(pad_w), int(dst_row_pitch), int(dst_image_rows))

@@ -52,9 +52,10 @@ def run(name, N, H, W, C, K, R, S, act, iters, image_rows=0, bias=True):
     del x, y
 
 
-def run_bwd(name, N, H, W, C, K, R, S, iters):
-    """wgrad and dgrad of the same layer: algorithmic bytes = dy read + x read (wgrad) / dy read + dx written (dgrad), bf16."""
-    P, Q = H - R + 1, W - S + 1
+def run_bwd(name, N, H, W, C, K, R, S, iters, stride=1, path="tc"):
+    """wgrad and dgrad of the same layer: algorithmic bytes = dy read + x read (wgrad) / dy read + dx written (dgrad), bf16.
+    stride: the window step (dy [N][(H-R)/stride+1][(W-S)/stride+1][K]); path "fma" selects the FMA-pipe reference kernels."""
+    P, Q = (H - R) // stride + 1, (W - S) // stride + 1
     xb = torch.randint(0, 0x3F80, (N, H, W, C), dtype=torch.int16, device="cuda")
     dyb = torch.randint(0, 0x3F80, (N, P, Q, K), dtype=torch.int16, device="cuda")
     dyb ^= (torch.randint(0, 2, (N, P, Q, K), dtype=torch.int16, device="cuda") << 15)      # random signs
@@ -63,8 +64,9 @@ def run_bwd(name, N, H, W, C, K, R, S, iters):
     dx = torch.empty((N, H, W, C), dtype=torch.int16, device="cuda")
     alg = N * (H * W * C + P * Q * K) * 2
     flops = 2.0 * N * P * Q * K * R * S * C
-    for what, fn in (("wgrad", lambda: eng.conv_wgrad(xb, dyb, dw, N, H, W, C, K, R, S)),
-                     ("dgrad", lambda: eng.conv_dgrad(dyb, f, dx, N, H, W, C, K, R, S))):
+    eng.conv_bwd_select(reference=(path == "fma"))
+    for what, fn in (("wgrad", lambda: eng.conv_wgrad(xb, dyb, dw, N, H, W, C, K, R, S, stride=stride)),
+                     ("dgrad", lambda: eng.conv_dgrad(dyb, f, dx, N, H, W, C, K, R, S, stride=stride))):
         for _ in range(3):
             fn()
         torch.cuda.synchronize()
@@ -80,7 +82,8 @@ def run_bwd(name, N, H, W, C, K, R, S, iters):
         ms = e0.elapsed_time(e1) / iters
         print(json.dumps({"case": name + " " + what, "host_enqueue_us": host_us, "N": N, "ms": ms, "img_per_s": N / (ms * 1e-3), "alg_GBps": alg / (ms * 1e-3) / 1e9,
                           "hbm_frac": alg / (ms * 1e-3) / 1e9 / HBM, "useful_TFLOPs": flops / (ms * 1e-3) / 1e12,
-                          "path": os.environ.get("PCNN_CONV_BWD", "tc"), "working_set_MB": alg / 1e6}), flush=True)
+                          "path": path, "stride": stride, "working_set_MB": alg / 1e6}), flush=True)
+    eng.conv_bwd_select(reference=False)
     del xb, dyb, dx
 
 
@@ -92,6 +95,18 @@ if only == "bwdpad":                                                   # filter 
     run_bwd("224x224x3->16x3x3 bf16 (padded to 64 filters)", 128, 224, 224, 3, 16, 3, 3, 10)
 if only == "bwdk128":                                                  # 128 filters: two 64-filter groups per dy row
     run_bwd("224x224x3->128x3x3 bf16", 64, 224, 224, 3, 128, 3, 3, 10)
+if only == "bwds":                                                     # strided backward passes (config 5 at stride 2) next to stride 1
+    import subprocess
+    q = subprocess.run(["nvidia-smi", "--id=%d" % torch.cuda.current_device(), "--query-gpu=name,power.limit,clocks.max.sm",
+                        "--format=csv,noheader"], capture_output=True, text=True).stdout.strip()
+    print(json.dumps({"case": "device", "torch_name": torch.cuda.get_device_name(), "nvidia_smi_name_power_limit_max_sm_clock": q,
+                      "hbm_peak_GBps_used_for_hbm_frac": HBM}), flush=True)
+    for N in (32, 128):
+        run_bwd("224x224x3->64x3x3/2 bf16 (config 5, stride 2)", N, 224, 224, 3, 64, 3, 3, 10, stride=2)
+    run_bwd("224x224x3->64x3x3/2 bf16 (config 5, stride 2)", 8, 224, 224, 3, 64, 3, 3, 2, stride=2, path="fma")
+    for N in (32, 128):
+        run_bwd("224x224x3->64x3x3 bf16 (config 5)", N, 224, 224, 3, 64, 3, 3, 10)
+    run_bwd("224x224x3->64x3x3 bf16 (config 5)", 8, 224, 224, 3, 64, 3, 3, 2, path="fma")
 if only == "bwd128":                                                   # the profiler's target: few launches
     run_bwd("224x224x3->64x3x3 bf16 (config 5)", 128, 224, 224, 3, 64, 3, 3, 2)
 if only in ("all", "lenet"):
